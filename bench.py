@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W              # our arm (CUDA, sm_100a), BASELINE config 2
     python bench.py --config 4|5 --gpus N ...                  # the other single-path configs (extra lines)
     python bench.py --impl reference --steps K --warmup W      # reference arm (CPU restatement)
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs, DIR/*.npy
 
 A "step" is one pass of the hot path over one batch: posterior + qLogEI + global arg-max over the rank's
 candidate shard (config 2: 1,000,000 x 20 rows, n=256 training points, Matern-5/2 ARD, S=512 Sobol base
@@ -334,7 +335,8 @@ def run_b200(args):
     best_val, best_idx = unpack_best(int(key_host.item()))
     e2e_ms = timed(step_e2e, steps, warmup, idle_start=True)
     key_coded = int(key_host.item())
-    e2e32_ms = timed(step_e2e_f32, max(3, steps // 4), 2, idle_start=True) / max(3, steps // 4)
+    e2e32_ms = timed(step_e2e_f32, steps, 2, idle_start=True) / steps
+    key_f32 = int(key_host.item())
     gp.check_host_pass()
     if peer is not None:
         peer.check()
@@ -422,6 +424,13 @@ def run_b200(args):
         }
         if strong is not None:
             line["strong_scaling"] = strong
+        if args.dump_outputs:
+            outs = {"best_value": best_val, "best_index": best_idx}
+            outs["e2e_best_value"], outs["e2e_best_index"] = unpack_best(key_coded)
+            outs["e2e_f32_best_value"], outs["e2e_f32_best_index"] = unpack_best(key_f32)
+            if strong is not None:
+                outs["strong_best_value"], outs["strong_best_index"] = strong["best"]["value"], strong["best"]["index"]
+            _dump_outputs(args.dump_outputs, outs)
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -502,6 +511,7 @@ def run_other(args):
         dist.barrier()  # data generation differs per rank by seconds; the peer reduction waits ~11 s at most
     with ClockSampler(local_rank) as clocks:
         total_ms = timed(step, steps, warmup)
+    best_val, best_idx = unpack_best(int(key_host.item()))
     kern_ms = timed(kernel_fn, steps, 2) / steps
     topk = None
     if args.config == 5:
@@ -525,11 +535,25 @@ def run_other(args):
                          "unit": "TFLOP/s", "frac": achieved / peaks["bf16_tflops"], "traffic": None,
                          "kernel_ms": kern_ms, "peak_source": peaks["source"], "note": rl_note},
             "cpu_baseline": None,
-            "notes": {"best": dict(zip(("value", "index"), unpack_best(int(key_host.item())))), "topk": topk},
+            "notes": {"best": {"value": best_val, "index": best_idx}, "topk": topk},
         }
+        if args.dump_outputs:
+            _dump_outputs(args.dump_outputs, {"best_value": best_val, "best_index": best_idx})
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def _dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write what the timed path returned in its last step as ``out_dir/<name>.npy`` (float64: every value here,
+    indices included, is exact in it).  The inputs are seeded, so two builds run with the same arguments can be
+    compared output for output."""
+    import numpy as np
+
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.asarray(a, dtype=np.float64))
 
 
 def _emit(line: dict) -> None:
@@ -568,15 +592,18 @@ def run_hybrid(args):
     rows_per_step = 16 * (len(disc) * min(search.n_sobol, search.max_rows // len(disc))
                           + search.n_rounds * search.n_seeds * search.n_local)
     cb = np.array([[0.0] * d_cont, [1.0] * d_cont])
-    steps, warmup = max(1, min(args.steps, 5)), 1
+    steps, warmup = args.steps, 1
+    last = {}
 
     def step():
-        return hy.recommend_hybrid(gp, acq, disc, cb, 16, None, S, 3, search)
+        last["out"] = hy.recommend_hybrid(gp, acq, disc, cb, 16, None, S, 3, search)
 
     timed = _Timer(dev, world)
     with ClockSampler(local_rank) as clocks:
         ms = timed(step, steps, warmup) / steps
-    pts, idx, value = step()
+    pts, idx, value = last["out"]
+    if args.dump_outputs:
+        _dump_outputs(args.dump_outputs, {"points": pts, "configuration_index": idx, "joint_qnei": value})
     _emit({
         "metric": "candidates/sec scored (qNEI S=512, hybrid 8 discrete x 4 continuous, q=16 batch)",
         "value": rows_per_step / (ms * 1e-3), "unit": UNIT, "n_gpus": 1, "steps": steps, "warmup": warmup,
@@ -605,7 +632,13 @@ def main():
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--config", type=int, choices=[2, 3, 4, 5], default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm")
     if args.impl == "reference":
         run_reference(args)
     elif args.config == 2:

@@ -1,7 +1,8 @@
 """The reference's own ``Campaign`` driving ``B200BotorchRecommender`` (baybe_b200/baybe_plugin.py), unmodified.
 
-``baybe`` is imported from ``/root/reference`` (or ``baseline/_ref`` when present); its un-installable dependency
-``cattrs`` is replaced by the book-keeping stand-in in ``tests/shims`` (serialisation is not on this path).
+``baybe`` is imported from ``oracle/_ref`` (installed there by ``build()``, see ``oracle/install_reference.sh``);
+its un-installable dependency ``cattrs`` is replaced by the book-keeping stand-in in ``tests/shims``
+(serialisation is not on this path).
 Without a GPU the engine is replaced by ``tests.helpers.OracleBackedGP`` (same interface, float64 oracle on the
 CPU): what is checked HERE is the binding -- subclass gates, hook signature, metadata masks ->
 ``FilteredSubspaceDiscrete`` -> position masks, index plumbing, pending experiments, subset-generating
@@ -18,7 +19,7 @@ import pandas as pd
 import pytest
 
 ROOT = Path(__file__).resolve().parents[1]
-REF = next((p for p in (ROOT / "baseline" / "_ref", Path("/root/reference")) if (p / "baybe").is_dir()), None)
+REF = ROOT / "oracle" / "_ref" if (ROOT / "oracle" / "_ref" / "baybe").is_dir() else None
 pytestmark = pytest.mark.skipif(REF is None, reason="the reference package (baybe) is not available on this box")
 
 

@@ -1,7 +1,7 @@
 """The real ``Campaign`` -> ``B200BotorchRecommender`` flow of tests/test_campaign_binding.py on the CUDA engine
-(no stand-in: ``torch.cuda.is_available()`` keeps ``DeviceGP``).  ``baybe`` comes from ``baseline/_ref`` (the
-offline ``pip install --no-deps --target`` of the reference, which travels to the GPU box) with the cattrs
-stand-in of ``tests/shims``; skipped when the reference package is not on the box."""
+(no stand-in: ``torch.cuda.is_available()`` keeps ``DeviceGP``).  ``baybe`` comes from ``oracle/_ref`` (the
+copy of the unmodified reference package that ``build()`` makes) with the cattrs
+stand-in of ``tests/shims``; skipped when the reference package is not installed there."""
 from __future__ import annotations
 
 import pytest

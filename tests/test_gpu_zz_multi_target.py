@@ -1,6 +1,6 @@
 """Round-2 additions that run LAST in the GPU suite (the driver runs it with ``-x``): the multi-target surrogate
 flow and the hybrid-space flow of tests/test_campaign_binding.py on the CUDA engine, under the reference's real
-``Campaign`` (``baseline/_ref``); skipped when the reference package is not on the box."""
+``Campaign`` (``oracle/_ref``); skipped when the reference package is not on the box."""
 from __future__ import annotations
 
 import numpy as np
